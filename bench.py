@@ -10,6 +10,7 @@ K timed steps the driver asks for cover more than a second of device time.
   python bench.py --gpus N --steps K --warmup W            our CUDA path: device-resident `value`, host-buffer `e2e`,
                                                            plus a `configs` block with the other BASELINE configurations
   python bench.py --impl reference ...                     the CPU restatement of the reference chain (oracle port)
+  python bench.py ... --dump-outputs DIR                   also writes what the timed path computed to DIR/*.npy (dump_outputs)
 
 Prints ONE JSON line (rank 0).  The CPU oracle is used here only as the checker (parity spot checks on the very buffers
 that were timed) and as the timed CPU baseline; nothing on the GPU arm's timed path touches it.
@@ -272,6 +273,29 @@ def rx_stage_ms(L, blk, names=("stage1_fir", "chan_filter", "demod_or_loop", "sy
         L.qrl_rx_profile_read(blk._h, s, Ct.byref(m), Ct.byref(n))
         out[name] = (m.value, n.value)
     return out
+
+
+DUMP_BUDGET = 63 << 20      # array bytes; the .npy headers, counts and channel list stay inside the last MB of 64 MB
+
+
+def dump_outputs(blk, out_dir):
+    """What the step's last qrl_rx_work call left on every output port, i.e. what read_port() hands a caller (each call replaces
+    the ports; the state carried from all earlier calls is in them), as float32 DIR/port<p>.npy: the channels' items back to back,
+    [items] for bit and float ports, [items, 2] (I, Q) for complex ones; DIR/counts.npy (float64 [ports, channels]) holds each
+    channel's item count, so channel i of port p is the counts[p, i] items after the first sum(counts[p, :i]).  Channels whose ports
+    do not all fit DUMP_BUDGET are left out by a fixed seeded draw; DIR/channels.npy lists the ones written."""
+    ports = [blk.read_port(p) for p in range(blk.nports)]
+    C = blk.n_channels
+    bytes_per_channel = sum(max(len(v) for v in port) * (8 if port[0].dtype == np.complex64 else 4) for port in ports)
+    n_keep = min(C, DUMP_BUDGET // max(1, bytes_per_channel))
+    chans = np.arange(C) if n_keep == C else np.sort(np.random.default_rng(0).choice(C, n_keep, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "channels.npy"), chans.astype(np.float64))
+    np.save(os.path.join(out_dir, "counts.npy"), np.array([[len(port[c]) for c in chans] for port in ports], np.float64))
+    for p, port in enumerate(ports):
+        a = np.concatenate([port[c] for c in chans])
+        a = a.view(np.float32).reshape(-1, 2) if a.dtype == np.complex64 else a.astype(np.float32)
+        np.save(os.path.join(out_dir, "port%d.npy" % p), a)
 
 
 def parity_bits(blk, X, oracle_kind, oracle_args, channels, port=2, float_port=0):
@@ -836,6 +860,8 @@ def run_ours(args):
     ms_max = float(t_ms.item())
     n_calls = args.steps * CALLS_PER_STEP
     value = world * C * T * n_calls / (ms_max * 1e-3) / 1e6
+    if args.dump_outputs and rank == 0:
+        dump_outputs(blk, args.dump_outputs)
 
     # ---- e2e: the reference-facing call with HOST buffers: H2D of the gr_complex slab + D2H of the decoded bits, every call
     old_aff, numa = bind_to_gpu_numa(torch, local)
@@ -1099,6 +1125,8 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline legs (profiling runs)")
     ap.add_argument("--no-parity", action="store_true", help="skip the full-size parity spot checks")
     ap.add_argument("--headline-only", action="store_true", help="config 2 only (no `configs` block)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the output ports of the timed path's last "
+                    "call to DIR/*.npy (float32, rank 0, at most 64 MB; inputs are seeded, so runs with the same arguments compare)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

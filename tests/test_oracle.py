@@ -1,5 +1,5 @@
 """CPU tier: pin the ORACLE itself (the known-answer tests the reference never had, SURVEY.md section 4 / 8c)."""
-import ctypes as C
+import json
 import os
 
 import numpy as np
@@ -75,17 +75,14 @@ def test_sincos_and_atan(oracle):
 
 
 def test_deemph_taps_against_compiled_reference(oracle):
-    """oracle/_ref = /root/reference/src/gr/emphasis.cpp compiled as-is (the only stand-alone piece)."""
-    so = os.path.join(ROOT, "oracle", "_ref", "libqrl_ref_emphasis.so")
-    if not os.path.exists(so):
-        pytest.skip("oracle/_ref not built (reference tree absent)")
-    R = C.CDLL(so)
+    """The taps of the reference's src/gr/emphasis.cpp compiled as-is (the only stand-alone piece, oracle/_ref), as frozen in
+    tests/golden/golden_v1.json by tests/golden/make_golden.py."""
+    G = json.load(open(os.path.join(ROOT, "tests", "golden", "golden_v1.json")))["emphasis"]
     for fs, tau in ((20000, 50e-6), (8000, 50e-6), (48000, 75e-6)):
-        a = np.zeros(2); b = np.zeros(2)
-        R.ref_deemph_taps(C.c_int(fs), C.c_double(tau), a.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p))
+        a, b = np.array([float.fromhex(v) for v in G["deemph_%d_%g" % (fs, tau)]]).reshape(2, 2)
         oa, ob = oracle.deemph_taps(fs, tau)
         assert np.array_equal(a, oa) and np.array_equal(b, ob)
-        R.ref_preemph_taps(C.c_int(fs), C.c_double(tau), C.c_double(-1.0), a.ctypes.data_as(C.c_void_p), b.ctypes.data_as(C.c_void_p))
+        a, b = np.array([float.fromhex(v) for v in G["preemph_%d_%g" % (fs, tau)]]).reshape(2, 2)
         oa, ob = oracle.preemph_taps(fs, tau)
         assert np.array_equal(a, oa) and np.array_equal(b, ob)
 

@@ -1,47 +1,44 @@
-"""Pins the oracle (and the host-side sink restatements) to REFERENCE CODE: oracle/_ref/libqrl_ref_blocks.so is
-/root/reference/src/gr/{gr_4fsk_discriminator, gr_deframer_bb, gr_bit_sink, gr_audio_sink, gr_const_sink, dsss_encoder_bb_impl,
-dsss_decoder_cc_impl, cessb/clipper_cc_impl, cessb/stretcher_cc_impl} compiled UNMODIFIED against the runtime stand-in in
-oracle/gr_stub/ (oracle/Makefile target `ref`; oracle/ref_blocks_shim.cpp plays the scheduler).  CPU tier."""
+"""Pins the oracle (and the host-side sink restatements) to REFERENCE CODE: tests/golden/ref_blocks_v1.json and
+ref_cessb_clipper_v1.npy hold what the reference's src/gr/{gr_4fsk_discriminator, gr_deframer_bb, gr_bit_sink, gr_audio_sink,
+gr_const_sink, gr_sample_sink, gr_zero_idle_bursts, rx_fft, dsss_decoder_cc_impl, rssi_tag_block, cessb/clipper_cc_impl,
+cessb/stretcher_cc_impl}, compiled UNMODIFIED against the runtime stand-in in oracle/gr_stub/ (oracle/Makefile target `ref`;
+oracle/ref_blocks_shim.cpp plays the scheduler), returned for the seeded inputs and call schedules of tests/golden/ref_cases.py
+(tests/golden/make_ref_golden.py).  CPU tier."""
 import ctypes as C
+import importlib
+import json
+import os
 
 import numpy as np
 import pytest
 
 from oracle import oracle as O
+from tests.golden import ref_cases as RC
+from tests.golden.ref_cases import sha
+
+GOLDEN = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+G = json.load(open(os.path.join(GOLDEN, "ref_blocks_v1.json")))
 
 
 def _p(a):
     return a.ctypes.data_as(C.c_void_p)
 
 
-@pytest.fixture(scope="module")
-def R():
-    r = O.ref_blocks()
-    if r is None:
-        pytest.skip("oracle/_ref/libqrl_ref_blocks.so not built (reference tree absent and no prebuilt copy)")
-    return r
-
-
-def test_discriminator_is_the_reference_block(R):
-    rng = np.random.default_rng(11)
-    n = 20000
-    m = rng.random((4, n)).astype(np.float32)
-    m[:, :2000] = np.round(m[:, :2000] * 4) / 4          # many exact ties: the strict-greater rule decides
-    m[:, 2000:2100] = 0.0
-    ref = np.zeros(2 * n, np.float32); got = np.zeros(2 * n, np.float32)
-    R.ref_disc4(_p(m[0]), _p(m[1]), _p(m[2]), _p(m[3]), n, _p(ref))
+def test_discriminator_is_the_reference_block():
+    m = RC.disc4_input()
+    n = m.shape[1]
+    got = np.zeros(2 * n, np.float32)
     O.lib().qo_disc4(_p(m[0]), _p(m[1]), _p(m[2]), _p(m[3]), n, _p(got))
-    assert np.array_equal(ref, got)
-    assert np.any(ref == 0.0) and len(np.unique(ref)) == 3      # -0.707107, 0, +0.707107 all occur
+    assert len(got) == G["disc4"]["n"] and sha(got) == G["disc4"]["sha256"]
+    assert np.any(got == 0.0) and len(np.unique(got)) == 3      # -0.707107, 0, +0.707107 all occur
 
 
-def test_cessb_clipper_against_the_reference_block(R):
-    rng = np.random.default_rng(12)
-    n = 8 * 1024
-    x = ((rng.standard_normal(n) + 1j * rng.standard_normal(n)) * rng.choice([0.05, 0.5, 1.5], n)).astype(np.complex64)
-    x[:16] = 0
-    ref = np.zeros(n, np.complex64); got = np.zeros(n, np.complex64)
-    assert R.ref_cessb_clipper(_p(x), n, 0.95, _p(ref)) == n
+def test_cessb_clipper_against_the_reference_block():
+    x = RC.cessb_clipper_input()
+    n = len(x)
+    ref = np.load(os.path.join(GOLDEN, "ref_cessb_clipper_v1.npy"))
+    assert G["cessb_clipper"]["returned"] == n and ref.shape == (n,) and ref.dtype == np.complex64
+    got = np.zeros(n, np.complex64)
     O.lib().qo_cessb_clipper(_p(x), n, C.c_float(0.95), _p(got))
     # magnitude path (sqrt, min) is IEEE on both sides; the phase goes through cos / sin, libm (VOLK generic) in the compiled
     # reference vs the oracle's fixed polynomial: 3e-7 each (tests/test_oracle.py::test_sincos_and_atan)
@@ -52,243 +49,153 @@ def test_cessb_clipper_against_the_reference_block(R):
 
 
 @pytest.mark.parametrize("chunk", [1024, 3072])
-def test_cessb_stretcher_is_the_reference_block_bit_for_bit(R, chunk):
-    rng = np.random.default_rng(13)
-    n = 9 * 1024 + 2
-    x = ((rng.standard_normal(n) + 1j * rng.standard_normal(n)) * rng.choice([0.1, 0.6, 1.2], n)).astype(np.complex64)
-    ref = np.zeros(n, np.complex64); got = np.zeros(n, np.complex64)
-    n_ref = R.ref_cessb_stretcher(_p(x), n, chunk, _p(ref))
+def test_cessb_stretcher_is_the_reference_block_bit_for_bit(chunk):
+    x = RC.cessb_stretcher_input()
+    n = len(x)
+    want = G["cessb_stretcher"][str(chunk)]
+    got = np.zeros(n, np.complex64)
     n_got = O.lib().qo_cessb_stretcher(_p(x), n, _p(got))
+    n_ref = want["n"]
     assert n_got == n - 2 and n_ref == 9 * 1024
-    assert np.array_equal(ref[:n_ref].view(np.float32), got[:n_ref].view(np.float32))      # chunking of the reference block is invisible
+    assert sha(got[:n_ref]) == want["sha256"]                    # the reference block, in either chunking, gave these bits
     assert np.any(np.abs(got[:n_ref]) < np.abs(x[:n_ref]) * 0.9)                           # the stretcher did act
 
 
-def _planted_bits(rng, n, words):
-    bits = rng.integers(0, 2, n, dtype=np.uint8)
-    pos = 50
-    while pos + 500 < n:
-        w, nb = words[int(rng.integers(0, len(words)))]
-        bits[pos:pos + nb] = [(w >> (nb - 1 - k)) & 1 for k in range(nb)]
-        pos += int(rng.integers(100, 700))
-    return bits
-
-
 @pytest.mark.parametrize("modem_type", [1, 2, 3])
-def test_gr_deframer_bb_is_the_reference_block(R, modem_type):
-    rng = np.random.default_rng(20 + modem_type)
-    words = [(0xED89, 16), (0x89ED, 16), (0x98DE, 16), (0xED77, 16), (0x8CC8, 16), (0x4C8A2B, 24), (0xB5, 8)]
-    bits = _planted_bits(rng, 60000, words)
-    h = R.ref_dfbb_create(modem_type)
+def test_gr_deframer_bb_is_the_reference_block(modem_type):
     d = O.DeframerBB(modem_type)
-    ref, got = [], []
-    pos = 0
-    while pos < len(bits):
-        m = int(rng.integers(1, 3000))
-        chunk = np.ascontiguousarray(bits[pos:pos + m]); pos += m
-        out = np.zeros(4 * len(chunk) + 64, np.uint8)
-        k = R.ref_dfbb_work(h, _p(chunk), len(chunk), _p(out), len(out))
-        ref.append(out[:k].copy()); got.append(d.work(chunk))
-    R.ref_block_destroy(h)
-    ref = np.concatenate(ref); got = np.concatenate(got)
-    assert len(ref) > 1000 and np.array_equal(ref, got)
+    got = np.concatenate([d.work(chunk) for chunk in RC.deframer_chunks(modem_type)])
+    want = G["deframer"][str(modem_type)]
+    assert len(got) > 1000 and len(got) == want["n"] and sha(got) == want["sha256"]
 
 
 @pytest.mark.parametrize("kind", ["bit", "audio", "const"])
-def test_sink_restatements_follow_the_reference_sinks(R, kind):
+def test_sink_restatements_follow_the_reference_sinks(kind):
     """qradiolink_b200.demod.gr_*_sink (what the Python host side polls) against the compiled gr_*_sink.cpp, random schedules."""
-    import importlib
     demod = importlib.import_module("qradiolink_b200.demod")
-    rng = np.random.default_rng({"bit": 31, "audio": 32, "const": 33}[kind])
     mine = getattr(demod, "gr_%s_sink" % kind)()
-    h = getattr(R, "ref_%s_sink_create" % kind)()
-    work, get = getattr(R, "ref_%s_sink_work" % kind), getattr(R, "ref_%s_sink_get" % kind)
-    dt = {"bit": np.uint8, "audio": np.float32, "const": np.complex64}[kind]
-    big = {"bit": 400000, "audio": 3000, "const": 120}[kind]
-    for step in range(400):
-        if rng.random() < 0.6:
-            n = int(rng.integers(0, big))
-            if kind == "bit":
-                x = rng.integers(0, 2, n, dtype=np.uint8)
-            elif kind == "audio":
-                x = rng.standard_normal(n).astype(np.float32)
-            else:
-                x = (rng.standard_normal(n) + 1j * rng.standard_normal(n)).astype(np.complex64)
-            assert work(h, _p(x), n) == mine.work(x)
+    want = G["sinks"][kind]
+    works, gets = iter(want["work"]), iter(want["get"])
+    for x in RC.sink_ops(kind):
+        if x is not None:
+            assert next(works) == mine.work(x)
         else:
-            out = np.zeros(1 << 21, dt) if kind == "bit" else np.zeros(1 << 14, dt)
-            k = get(h, _p(out), len(out))
+            k, digest = next(gets)
             m = mine.get_data()
             if k < 0:
                 assert m is None
             else:
-                assert m is not None and len(m) == k and np.array_equal(out[:k], m)
-    R.ref_block_destroy(h)
+                assert m is not None and len(m) == k and sha(m) == digest
+    assert next(works, None) is None and next(gets, None) is None
 
 
-def test_sample_sink_restatement_follows_the_reference_sink(R):
+def test_sample_sink_restatement_follows_the_reference_sink():
     """qradiolink_b200.demod.gr_sample_sink against the compiled gr_sample_sink.cpp: enable, window changes (odd sizes), the 524288-item
     drop rule, random schedules."""
-    import importlib
     demod = importlib.import_module("qradiolink_b200.demod")
-    rng = np.random.default_rng(34)
     mine = demod.gr_sample_sink()
-    h = R.ref_sample_sink_create()
-    out = np.zeros(1 << 20, np.complex64)
-    for step in range(300):
-        r = rng.random()
-        if step == 5:
-            R.ref_sample_sink_set_enabled(h, 1); mine.set_enabled(True)
-        if r < 0.55:
-            n = int(rng.integers(0, 200000))
-            x = (rng.standard_normal(n) + 1j * rng.standard_normal(n)).astype(np.complex64)
-            assert R.ref_sample_sink_work(h, _p(x), n) == mine.work(x)
-        elif r < 0.65:
-            w = int(rng.integers(1, 30000))
-            R.ref_sample_sink_set_window(h, w); mine.set_sample_window(w)
+    want = G["sample_sink"]
+    works, gets = iter(want["work"]), iter(want["get"])
+    for op in RC.sample_sink_ops():
+        if op[0] == "enable":
+            mine.set_enabled(True)
+        elif op[0] == "work":
+            assert next(works) == mine.work(op[1])
+        elif op[0] == "window":
+            mine.set_sample_window(op[1])
         else:
-            k = R.ref_sample_sink_get(h, _p(out), len(out))
+            k, digest = next(gets)
             m = mine.get_data()
             if k < 0:
                 assert m is None
             else:
-                assert m is not None and len(m) == k and np.array_equal(out[:k], m)
-    R.ref_block_destroy(h)
+                assert m is not None and len(m) == k and sha(m) == digest
+    assert next(works, None) is None and next(gets, None) is None
 
 
-def test_zero_idle_bursts_is_the_reference_block(R):
+def test_zero_idle_bursts_is_the_reference_block():
     """gr_zero_idle_bursts.cpp compiled unmodified (stream tags through the stand-in's get_tags_in_window): delay of history-1 items,
     a counter loaded `delay` items before the tagged one, later tags overriding a running count.  Tags are kept at least `delay`
     items inside their work() window -- the only place the restatement deviates (it also honours the ones the reference drops)."""
-    rng = np.random.default_rng(31)
-    n, delay = 30000, 62
-    x = (rng.standard_normal(n) + 1j * rng.standard_normal(n)).astype(np.complex64)
-    chunks = np.array([4096, 1000, 8192, 5000, 20000], np.int64)
-    edges = np.concatenate([[0], np.cumsum(chunks)])
-    tag_items, tag_vals = [], []
-    for k in range(len(chunks)):
-        lo, hi = edges[k], min(edges[k + 1], n)
-        if hi - lo < 400:
-            continue
-        for j in range(3):
-            tag_items.append(int(lo + delay + rng.integers(0, hi - lo - delay)))
-            tag_vals.append(int(rng.integers(1, 900)))
-    tag_items.append(tag_items[0] + 5); tag_vals.append(3)           # overrides a running count with a short one
-    tag_items.append(30); tag_vals.append(500)                        # item < delay: never matches
-    to = np.array(tag_items, np.int64); tv = np.array(tag_vals, np.int64)
-    ref = np.zeros(n, np.complex64)
-    ch = chunks.astype(np.int64)
-    done = R.ref_zero_idle(_p(x), n, delay, _p(to), _p(tv), len(to), _p(ch.astype(np.dtype("l"))), len(ch), _p(ref))
-    assert done == n
-    got = O.zero_idle(x, delay, to, tv)
-    assert np.array_equal(ref.view(np.uint32), got.view(np.uint32))
+    x, to, tv, _ = RC.zero_idle_input()
+    n = len(x)
+    got = O.zero_idle(x, RC.ZERO_IDLE_DELAYS[0], to, tv)
+    assert G["zero_idle"]["62"]["done"] == n and sha(got) == G["zero_idle"]["62"]["sha256"]
     assert np.count_nonzero(got == 0) > 1439 + 500 and np.all(got[:1439] == 0)
     nz = got[1439:] != 0
     assert np.array_equal(got[1439:][nz], x[:n - 1439][nz])              # what is not zeroed is the input, 1439 items late
     # delay = 0: no history, pure pass-through + tags at their own item
-    ref0 = np.zeros(n, np.complex64)
-    R.ref_zero_idle(_p(x), n, 0, _p(to), _p(tv), len(to), _p(ch.astype(np.dtype("l"))), len(ch), _p(ref0))
     got0 = O.zero_idle(x, 0, to, tv)
-    assert np.array_equal(ref0.view(np.uint32), got0.view(np.uint32))
+    assert G["zero_idle"]["0"]["done"] == n and sha(got0) == G["zero_idle"]["0"]["sha256"]
 
 
 @pytest.mark.parametrize("n_fft", [1024, 32768])
-def test_rx_fft_restatement_follows_the_reference_block(R, n_fft):
+def test_rx_fft_restatement_follows_the_reference_block(n_fft):
     """rx_fft.cpp compiled unmodified (FFTW replaced by the oracle's own DFT in the stand-in, so this pins the buffering, windowing,
     d_push drop rule, power-spectrum kernel and fft-shift, not FFTW's rounding): same points after every get, for ragged work()
     sizes incl. calls longer than the FFT, calls while a spectrum is pending, disable / enable and a change of size."""
-    rng = np.random.default_rng(61)
-    n = n_fft * 9 + 777
-    t = np.arange(n)
-    x = (0.3 * np.exp(2j * np.pi * 0.1234 * t) + 0.05 * (rng.standard_normal(n) + 1j * rng.standard_normal(n))).astype(np.complex64)
-    x[5000:5050] = 0
-    h = R.ref_rx_fft_create(n_fft, O.WIN_BLACKMAN_HARRIS)
     s = O.Spectrum(n_fft, O.WIN_BLACKMAN_HARRIS)
-    sizes = [n_fft // 3, 17, n_fft, n_fft // 2 + 5, 2 * n_fft + 9, 100, n_fft - 1, 3 * n_fft]
-    lo, k, got_any = 0, 0, 0
-    pts = np.empty(n_fft, np.float32)
-    for step, m in enumerate(sizes):
-        if step == 0:
-            R.ref_rx_fft_work(h, _p(x[lo:lo + 50]), 50); s.work(x[lo:lo + 50])      # not enabled yet: dropped
-            R.ref_rx_fft_set_enabled(h, 1); s.set_enabled(True)
-        m = min(m, n - lo)
-        R.ref_rx_fft_work(h, _p(x[lo:lo + m]), m); s.work(x[lo:lo + m]); lo += m
-        if step % 2 == 1:
-            nr = R.ref_rx_fft_get(h, _p(pts)); g = s.get()
-            assert (nr == 0) == (g is None), step
+    gets = iter(G["rx_fft"][str(n_fft)])
+    size, got_any = n_fft, 0
+    for op in RC.rx_fft_ops(n_fft):
+        if op[0] == "work":
+            s.work(op[1])
+        elif op[0] == "enable":
+            s.set_enabled(True)
+        elif op[0] == "size":
+            s.set_fft_size(op[1]); size = op[1]
+        elif op[0] == "drain":
+            s.get()
+        else:
+            nr, digest = next(gets)
+            g = s.get()
+            assert (nr == 0) == (g is None)
             if g is not None:
-                assert nr == n_fft and np.array_equal(pts.view(np.uint32), g.view(np.uint32)), step
-                got_any += 1
-                peak = int(np.argmax(g))
-                assert abs(peak - (n_fft // 2 + round(0.1234 * n_fft))) <= 1
-    assert got_any >= 3
-    R.ref_rx_fft_set_fft_size(h, n_fft // 2); s.set_fft_size(n_fft // 2)
-    R.ref_rx_fft_get(h, _p(pts)); s.get()
-    R.ref_rx_fft_work(h, _p(x[:n_fft]), n_fft); s.work(x[:n_fft])
-    nr = R.ref_rx_fft_get(h, _p(pts)); g = s.get()
-    assert nr == n_fft // 2 and np.array_equal(pts[:nr].view(np.uint32), g.view(np.uint32))
-    R.ref_block_destroy(h)
+                assert nr == size and len(g) == nr and sha(g) == digest
+                if size == n_fft:
+                    got_any += 1
+                    peak = int(np.argmax(g))
+                    assert abs(peak - (n_fft // 2 + round(RC.RX_FFT_FREQ * n_fft))) <= 1
+    assert next(gets, None) is None
+    assert got_any >= 3 and size == n_fft // 2 and g is not None                 # the last get came after the change of size
 
 
-BARKER_13 = np.array([1, 1, 1, 1, 1, 0, 0, 1, 1, 0, 1, 0, 1], np.int32)
-
-
-def test_dsss_decoder_restatement_is_the_reference_block(R):
+def test_dsss_decoder_restatement_is_the_reference_block():
     """dsss_decoder_cc_impl.cc compiled unmodified: the matched-filter taps its constructor builds, and general_work over a buffer laid
     out the way the restatement DEFINES the region in front of the declared history (the stream's own older items, zeros at the
     start): same symbols bit for bit, for several scheduler chunkings of the reference and several of the restatement."""
-    sps, N = 25, 325
-    h = R.ref_dsss_decoder_create(_p(BARKER_13), 13, C.c_float(sps))
-    assert R.ref_dsss_decoder_history(h) == N
+    want = G["dsss_decoder"]
+    sps, N = RC.DSSS_SPS, RC.DSSS_HISTORY
+    assert want["history"] == N
     nt = N + 11 * sps
-    tr = np.zeros(2 * nt, np.float32); tq = np.zeros(2 * nt, np.float32)
-    assert R.ref_dsss_decoder_taps(h, _p(tr), nt) == nt
-    O.lib().qo_dsss_decoder_taps(_p(BARKER_13), 13, sps, _p(tq))
-    assert np.array_equal(tr.view(np.uint32), tq.view(np.uint32))
-    rng = np.random.default_rng(71)
-    n_sym = 40
-    # a spread BPSK stream + noise so that the maximum is well defined, plus a stretch of exact zeros
-    chips = np.repeat(np.where(BARKER_13 > 0, 1.0, -1.0), sps)
-    bits = rng.integers(0, 2, n_sym) * 2 - 1
-    x = np.concatenate([b * chips for b in bits]).astype(np.complex64) * np.exp(0.4j).astype(np.complex64)
-    x = (x + 0.3 * (rng.standard_normal(len(x)) + 1j * rng.standard_normal(len(x)))).astype(np.complex64)
-    x[3000:3400] = 0
+    tq = np.zeros(2 * nt, np.float32)
+    O.lib().qo_dsss_decoder_taps(_p(RC.BARKER_13), 13, sps, _p(tq))
+    assert want["n_taps"] == nt and sha(tq) == want["taps_sha256"]
+    x, n_sym = RC.dsss_input()
     n = len(x)
     got = np.zeros(n_sym + 4, np.complex64)
     for chunk in (n, 1000, 77):
-        m = O.lib().qo_dsss_decoder_run(_p(BARKER_13), 13, sps, _p(x), n, chunk, _p(got), len(got))
+        m = O.lib().qo_dsss_decoder_run(_p(RC.BARKER_13), 13, sps, _p(x), n, chunk, _p(got), len(got))
         if chunk == n:
             first, m0 = got[:m].copy(), m
         assert m == m0 and np.array_equal(got[:m].view(np.uint32), first.view(np.uint32)), chunk
-    # reference: buffer = [2N - 1 zeros][x][slack]; output m is called with `in` = item m N - (N - 1) (history N), one or more per call
-    buf = np.concatenate([np.zeros(2 * N - 1, np.complex64), x, np.zeros(2 * N, np.complex64)])
-    for per_call in (1, 3, m0):
-        ref = np.zeros(m0, np.complex64)
-        done = 0
-        while done < m0:
-            k = min(per_call, m0 - done)
-            cons = C.c_long()
-            in_ptr = buf[(2 * N - 1) + done * N - (N - 1):]
-            out = np.zeros(k, np.complex64)
-            assert R.ref_dsss_decoder_work(h, _p(in_ptr), k, _p(out), C.byref(cons)) == k and cons.value == k * N
-            ref[done:done + k] = out; done += k
-        assert np.array_equal(ref.view(np.uint32), first.view(np.uint32)), per_call
+    # reference: fed one, three and all symbols' worth of input per general_work call
+    assert m0 == want["n_symbols"]
+    for per_call, digest in want["symbols_sha256"].items():
+        assert sha(first) == digest, per_call
     assert m0 >= n_sym - 2
-    R.ref_block_destroy(h)
 
 
-def test_rssi_tag_rule_is_the_reference_block(R):
+def test_rssi_tag_rule_is_the_reference_block():
     """rssi_tag_block.cpp compiled unmodified (add_item_tag through the stand-in): an "RSSI" tag every 300 items, value and offset, for
     several scheduler chunkings; the float accumulation order is the block's (sequential)."""
-    rng = np.random.default_rng(81)
-    n = 7000
-    x = ((rng.standard_normal(n) + 1j * rng.standard_normal(n)) * np.repeat(rng.uniform(1e-4, 2.0, n // 100), 100)).astype(np.complex64)
+    x = RC.rssi_input()
+    n = len(x)
     db_o = np.zeros(64, np.float32); at_o = np.zeros(64, np.int64)
     k = O.lib().qo_rssi_tags_run(_p(x), n, -3.5, _p(db_o), _p(at_o), 64)
     assert k == n // 300
-    for chunks in ([n], [299, 1, 300, 301, 5000, 2000], [7] * 1001):
-        ch = np.array(chunks, np.dtype("l"))
-        db_r = np.zeros(64, np.float32); at_r = np.zeros(64, np.int64)
-        kr = R.ref_rssi_tags(_p(x), n, C.c_float(-3.5), _p(ch), len(ch), _p(db_r), _p(at_r), 64)
-        assert kr == k and np.array_equal(at_r[:k], at_o[:k]) and np.array_equal(db_r[:k].view(np.uint32), db_o[:k].view(np.uint32)), chunks[:3]
+    assert len(G["rssi_tags"]) == len(RC.RSSI_CHUNKINGS)
+    for want in G["rssi_tags"]:
+        db_r = np.array([float.fromhex(v) for v in want["db"]], np.float32)
+        assert want["n"] == k and want["offsets"] == [int(v) for v in at_o[:k]] and np.array_equal(db_r.view(np.uint32), db_o[:k].view(np.uint32))
     assert np.array_equal(at_o[:k], np.arange(k) * 300 + 299)
