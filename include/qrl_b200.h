@@ -183,6 +183,29 @@ int  qrl_frontend_out_device(qrl_frontend*, float** data, long* stride, long* n_
 int  qrl_frontend_read(qrl_frontend*, float* dst /* [n_channels][cap] gr_complex */, long cap);
 long qrl_frontend_launch_count(const qrl_frontend*);
 
+/* ---- TX front end: 1 Msps -> device rate ------------------------------------------------------------------------------------------
+ * gr_mod_base (/root/reference/src/gr/gr_mod_base.cpp:38,211-290,799-805) always runs mod -> rotator_cc(2 pi offset / 1e6) and, when
+ * the sink runs at samp_rate >= 2 Msps, rational_resampler_ccf(N, 1, low_pass(N, samp_rate, 480000, 20000, BLACKMAN_HARRIS)) with
+ * N = samp_rate / 1e6 in front of the sink (below 2 Msps the rotator feeds the sink directly).  This object is that pair for a batch
+ * of channels: [n_channels][n] gr_complex at 1 Msps in (e.g. qrl_tx_out_device's buffer, on_device = 1), [n_channels][N n] items at
+ * samp_rate out.  Definition: tests/txfront_ref.py -- exact Q32 NCO with phase = base + inc (n - n_base), inc = rint(offset / 1e6 2^32),
+ * phase-continuous retunes; each output one sequential fma chain over the arm, oldest sample first.  Streaming: any chunking gives the
+ * same stream.  samp_rate is 1e6 or a multiple of 1e6 in [2e6, 56e6]; anything else is QRL_EINVAL.
+ * QRL_TXFRONT_SC16 stores per component (short) clamp(rintf(x * sc16_scale), -32768, 32767), interleaved I/Q: the arithmetic of a
+ * SIMD fc32 -> sc16 converter with UHD's scale 32767.  That is a definition chosen here (UHD's converter is not in the reference tree
+ * to pin it), like qrl_rx_work_sc16's.  It halves the HBM writes and the bytes that cross PCIe to the SDR. */
+enum { QRL_TXFRONT_FC32 = 0, QRL_TXFRONT_SC16 = 1 };
+typedef struct qrl_txfront qrl_txfront;
+int  qrl_txfront_create(int samp_rate /* 1e6, or a multiple of 1e6 in [2e6, 56e6] */, int n_channels, long max_in /* 1 Msps items per call */,
+                        int out_format, float sc16_scale, int device, qrl_txfront** out);
+int  qrl_txfront_destroy(qrl_txfront*);
+int  qrl_txfront_set_stream(qrl_txfront*, void* cuda_stream);
+int  qrl_txfront_set_carrier_offset(qrl_txfront*, int channel /* -1 = all */, double offset_hz);
+int  qrl_txfront_work(qrl_txfront*, const float* iq /* [C][stride] gr_complex at 1 Msps */, long n, long stride, int on_device, long* n_out);
+int  qrl_txfront_out_device(qrl_txfront*, void** data, long* stride, long* n_out);
+int  qrl_txfront_read(qrl_txfront*, void* dst /* [C][cap] items of the output format */, long cap);
+long qrl_txfront_launch_count(const qrl_txfront*);
+
 /* ---- design helpers (host only; the gr::filter::firdes calls the reference makes at construction /
  *      in set_filter_width, e.g. gr_demod_nbfm.cpp:82-90).  Return tap count or negative error. ---- */
 int qrl_firdes_low_pass(double gain, double fs, double fc, double tw, int window, float* out, int cap);

@@ -304,4 +304,45 @@ inline gr_mod_b200_sptr make_gr_mod_dmr(int sps = 125, int samp_rate = 1000000, 
                                         int n_channels = 1, long max_items = 4096, int device = 0)               // src/gr/gr_mod_dmr.h:37-38
 { return std::make_shared<gr_mod_b200>(QRL_MOD_DMR, sps, samp_rate, carrier_freq, filter_width, 0, n_channels, max_items, device); }
 
+// ---- TX front end: what gr_mod_base connects between the modulator and the SDR sink (gr_mod_base.cpp:38,211-290):
+// _rotator (set_carrier_offset, :799-805) and, at samp_rate >= 2 Msps, the xN _resampler.  1 Msps gr_complex in, samp_rate out,
+// as gr_complex (QRL_TXFRONT_FC32) or interleaved int16 I/Q (QRL_TXFRONT_SC16, per component clamp(rint(x * sc16_scale))).
+class tx_frontend_b200 {
+public:
+    tx_frontend_b200(int samp_rate, int n_channels = 1, long max_in = 1 << 20, int out_format = QRL_TXFRONT_FC32, float sc16_scale = 32767.0f, int device = 0)
+        : _C(n_channels), _N(samp_rate / 1000000), _fmt(out_format)
+    {
+        if (qrl_txfront_create(samp_rate, n_channels, max_in, out_format, sc16_scale, device, &_h) != QRL_OK)
+            throw std::runtime_error(std::string("qrl_txfront_create: ") + qrl_last_error(nullptr));
+    }
+    ~tx_frontend_b200() { qrl_txfront_destroy(_h); }
+    tx_frontend_b200(const tx_frontend_b200&) = delete;
+    tx_frontend_b200& operator=(const tx_frontend_b200&) = delete;
+    int set_carrier_offset(double offset_hz, int channel = -1) { return qrl_txfront_set_carrier_offset(_h, channel, offset_hz); }
+    int interpolation() const { return _N; }
+    // host path: [channels][stride] gr_complex at 1 Msps -> [channels][N n] items of the output format in `out` (fc32: 2 floats,
+    // sc16: 2 int16 per item); returns N n, or WORK_DONE on a shim error
+    template <class T>
+    int work(const gr_complex* in, long n, long stride, std::vector<T>& out)
+    {
+        static_assert(sizeof(T) == 8 || sizeof(T) == 4, "gr_complex or a pair of int16 per item");
+        long n_out = 0;
+        if ((sizeof(T) == 8) != (_fmt == QRL_TXFRONT_FC32)) return WORK_DONE;
+        if (qrl_txfront_work(_h, reinterpret_cast<const float*>(in), n, stride, 0, &n_out) != QRL_OK) return WORK_DONE;
+        out.resize(static_cast<size_t>(n_out) * _C);
+        if (n_out > 0 && qrl_txfront_read(_h, out.data(), n_out) != QRL_OK) return WORK_DONE;
+        return static_cast<int>(n_out);
+    }
+    // device path (e.g. the modulator's qrl_tx_out_device buffer): the output stays on the device, see out_device
+    long work_device(const float* d_in, long n, long stride)
+    {
+        long n_out = 0;
+        return qrl_txfront_work(_h, d_in, n, stride, 1, &n_out) == QRL_OK ? n_out : WORK_DONE;
+    }
+    int out_device(void** data, long* stride, long* n_out) { return qrl_txfront_out_device(_h, data, stride, n_out); }
+private:
+    qrl_txfront* _h = nullptr;
+    int _C, _N, _fmt;
+};
+
 }  // namespace qrl_gr

@@ -13,6 +13,6 @@ from .demod import (RxBlock, make_gr_demod_4fsk, make_gr_demod_qpsk, make_gr_dem
 from .mod import TxBlock, make_gr_mod_4fsk, make_gr_mod_qpsk, make_gr_mod_bpsk, make_gr_mod_2fsk, make_gr_mod_nbfm, make_gr_mod_ssb, make_gr_mod_gmsk, make_gr_mod_m17, make_gr_mod_dmr, make_gr_mod_dsss, make_gr_mod_am  # noqa: F401
 from .pfb import PfbChannelizer, PfbSynthesizer, mmdvm_port_map  # noqa: F401
 from .framing import Deframer, DeframerBB, MODE_FRAMING, SYNC_1K, SYNC_NARROW, SYNC_WIDE, SYNC_M17, frame  # noqa: F401
-from .frontend import Frontend  # noqa: F401
+from .frontend import Frontend, TxFrontend  # noqa: F401
 from .spectrum import Spectrum  # noqa: F401
 from .mmdvm import MmdvmDemod, MmdvmMod, MmdvmChannelsRx, MmdvmChannelsTx, mmdvm_tag_item  # noqa: F401

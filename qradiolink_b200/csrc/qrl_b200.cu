@@ -2877,6 +2877,182 @@ int qrl_frontend_read(qrl_frontend* h, float* dst, long cap)
 }
 long qrl_frontend_launch_count(const qrl_frontend* h) { return h ? h->launches : 0; }
 
+// ---------------------------------------------------------------------------------------------- TX front end (1 Msps -> device rate)
+namespace {
+constexpr int TXF_R = 8;                // outputs per thread and pass of txfront_interp_kernel
+constexpr int TXF_SMEM_MAX = 96 * 1024; // >= the 58 KB the kernel needs at 56 Msps
+}
+struct qrl_txfront : HandleBase {
+    int samp_rate = 0, N = 1, C = 0, fmt = QRL_TXFRONT_FC32, ntaps = 0, NTP = 0, H = 0, G = 1, P = 1, hist_cur = 0;
+    float scale = 32767.0f;
+    long max_in = 0;
+    size_t smem = 0;
+    float* d_taps = nullptr;                // [NTP][N] chain order
+    float2* d_hist[2] = { nullptr, nullptr };
+    float2* d_in = nullptr; void* d_out = nullptr; long long out_stride = 0; long n_out_last = 0;
+    long long n_in = 0;
+    std::vector<RotState> rot; RotState* d_rot = nullptr; bool rot_active = false;
+    size_t item_bytes() const { return fmt == QRL_TXFRONT_SC16 ? sizeof(short2) : sizeof(float2); }
+};
+
+int qrl_txfront_destroy(qrl_txfront* h)
+{
+    if (!h) return QRL_OK;
+    cudaSetDevice(h->device);
+    if (h->stream) cudaStreamSynchronize(h->stream);
+    for (void* p : h->allocs) cudaFree(p);
+    if (h->own_stream && h->stream) cudaStreamDestroy(h->stream);
+    delete h;
+    return QRL_OK;
+}
+int qrl_txfront_create(int samp_rate, int n_channels, long max_in, int out_format, float sc16_scale, int device, qrl_txfront** out)
+{
+    if (!out || n_channels <= 0 || max_in <= 0 || (out_format != QRL_TXFRONT_FC32 && out_format != QRL_TXFRONT_SC16)) {
+        set_err(nullptr, "qrl_txfront_create: bad argument"); return QRL_EINVAL;
+    }
+    if (samp_rate != 1000000 && (samp_rate < 2000000 || samp_rate > 56000000 || samp_rate % 1000000)) {
+        set_err(nullptr, "qrl_txfront_create: samp_rate " + std::to_string(samp_rate) + " is not supported (1e6, or a multiple of 1e6 in [2e6, 56e6])");
+        return QRL_EINVAL;
+    }
+    *out = nullptr;
+    if (qrl_device_count() <= device) { set_err(nullptr, "qrl_txfront_create: no CUDA device (this library has no CPU fallback)"); return QRL_ENODEV; }
+    qrl_txfront* h = new qrl_txfront();
+    h->samp_rate = samp_rate; h->N = samp_rate / 1000000; h->C = n_channels; h->max_in = max_in; h->device = device;
+    h->fmt = out_format; h->scale = sc16_scale;
+    auto fail = [&](int rc) { std::string e = h->err; qrl_txfront_destroy(h); g_err = e; return rc; };
+    if (cudaSetDevice(device) != cudaSuccess) { set_err(h, "cudaSetDevice failed"); return fail(QRL_ECUDA); }
+    if (cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking) != cudaSuccess) { set_err(h, "stream create failed"); return fail(QRL_ECUDA); }
+    h->own_stream = true;
+    int rc = upload_tables(h);
+    if (rc) return fail(rc);
+    if (h->N > 1) {
+        // gr_mod_base.cpp:211-258: rational_resampler_ccf(N, 1, low_pass(N, samp_rate, 480000, 20000, BLACKMAN_HARRIS))
+        const std::vector<float> taps = low_pass(h->N, samp_rate, 480000, 20000, WIN_BLACKMAN_HARRIS);
+        const int N = h->N;
+        h->ntaps = static_cast<int>(taps.size());
+        const int nt = (h->ntaps + N - 1) / N;
+        h->NTP = (nt + TXF_R - 1) / TXF_R * TXF_R;
+        h->H = h->NTP - 1;
+        std::vector<float> chain(static_cast<size_t>(h->NTP) * N, 0.0f);    // row i = step i of the chain: arm tap k = NTP - 1 - i
+        for (int i = 0; i < h->NTP; i++)
+            for (int p = 0; p < N; p++) {
+                const long j = p + static_cast<long>(h->NTP - 1 - i) * N;
+                if (j < h->ntaps) chain[static_cast<size_t>(i) * N + p] = taps[j];
+            }
+        if ((rc = upload_floats(h, &h->d_taps, chain))) return fail(rc);
+        h->G = 256 / N;
+        h->P = std::max(1, 1024 / (h->G * TXF_R));
+        h->smem = sizeof(float) * ((h->NTP * N + 1) & ~1) + sizeof(float2) * (h->G * TXF_R * h->P + h->NTP - 1);
+        if (h->smem > static_cast<size_t>(TXF_SMEM_MAX)) { set_err(h, "qrl_txfront_create: filter too long for the kernel's shared memory"); return fail(QRL_EINVAL); }
+        if (cudaFuncSetAttribute(txfront_interp_kernel<TXF_R, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TXF_SMEM_MAX) != cudaSuccess ||
+            cudaFuncSetAttribute(txfront_interp_kernel<TXF_R, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TXF_SMEM_MAX) != cudaSuccess) {
+            set_err(h, "qrl_txfront_create: cudaFuncSetAttribute failed"); return fail(QRL_ECUDA);
+        }
+        if ((rc = dev_alloc(h, &h->d_hist[0], static_cast<size_t>(h->H) * h->C))) return fail(rc);
+        if ((rc = dev_alloc(h, &h->d_hist[1], static_cast<size_t>(h->H) * h->C))) return fail(rc);
+    }
+    h->out_stride = static_cast<long long>(max_in) * h->N;
+    {
+        unsigned char* o = nullptr;
+        if ((rc = dev_alloc(h, &o, h->item_bytes() * static_cast<size_t>(h->out_stride) * h->C, false))) return fail(rc);
+        h->d_out = o;
+    }
+    if ((rc = dev_alloc(h, &h->d_rot, h->C))) return fail(rc);
+    h->rot.assign(h->C, RotState{ 0u, 0u, 0 });
+    if (cudaStreamSynchronize(h->stream) != cudaSuccess) { set_err(h, "create sync failed"); return fail(QRL_ECUDA); }
+    *out = h;
+    return QRL_OK;
+}
+int qrl_txfront_set_stream(qrl_txfront* h, void* s)
+{
+    if (!h) return QRL_EINVAL;
+    CK(cudaStreamSynchronize(h->stream));
+    if (h->own_stream && h->stream) { cudaStreamDestroy(h->stream); h->own_stream = false; }
+    if (s) h->stream = static_cast<cudaStream_t>(s);
+    else { CK(cudaStreamCreateWithFlags(&h->stream, cudaStreamNonBlocking)); h->own_stream = true; }
+    return QRL_OK;
+}
+int qrl_txfront_set_carrier_offset(qrl_txfront* h, int channel, double offset_hz)
+{
+    // gr_mod_base::set_carrier_offset (:799-805): rotator phase increment 2 pi offset / 1e6, at 1 Msps in front of the resampler
+    if (!h || channel < -1 || channel >= h->C) return QRL_EINVAL;
+    const unsigned inc = static_cast<unsigned>(static_cast<int>(static_cast<long long>(std::rint(offset_hz / 1e6 * 4294967296.0))));
+    for (int c = 0; c < h->C; c++) {
+        if (channel >= 0 && c != channel) continue;
+        RotState& r = h->rot[c];
+        r.base = r.base + r.inc * static_cast<unsigned>(h->n_in - r.n_base);
+        r.n_base = h->n_in;
+        r.inc = inc;
+    }
+    h->rot_active = false;
+    for (auto& r : h->rot) if (r.inc != 0 || r.base != 0) h->rot_active = true;
+    CK(cudaStreamSynchronize(h->stream));
+    CK(cudaMemcpy(h->d_rot, h->rot.data(), sizeof(RotState) * h->C, cudaMemcpyHostToDevice));
+    return QRL_OK;
+}
+int qrl_txfront_work(qrl_txfront* h, const float* iq, long n, long stride, int on_device, long* n_out)
+{
+    if (!h || !iq || n < 0 || stride < n) return QRL_EINVAL;
+    if (n > h->max_in) { set_err(h, "qrl_txfront_work: n exceeds max_in given at create"); return QRL_ERANGE; }
+    h->n_out_last = 0;
+    if (n_out) *n_out = 0;
+    if (n == 0) return QRL_OK;
+    CK(cudaSetDevice(h->device));
+    if (on_device) { int rc = check_device_ptr(h, iq, "qrl_txfront_work"); if (rc) return rc; }
+    const float2* x = reinterpret_cast<const float2*>(iq);
+    long long xstride = stride;
+    if (!on_device) {
+        if (!h->d_in) { int rc = dev_alloc(h, &h->d_in, static_cast<size_t>(h->max_in) * h->C, false); if (rc) return rc; }
+        CK(cudaMemcpy2DAsync(h->d_in, sizeof(float2) * h->max_in, iq, sizeof(float2) * stride, sizeof(float2) * n, h->C, cudaMemcpyHostToDevice, h->stream));
+        x = h->d_in; xstride = h->max_in;
+    }
+    const RotState* rs = h->rot_active ? h->d_rot : nullptr;
+    const bool sc16 = h->fmt == QRL_TXFRONT_SC16;
+    if (h->N == 1) {
+        dim3 g(static_cast<unsigned>(std::min<long>((n + 255) / 256, 4096)), h->C);
+        if (sc16) txfront_rot_kernel<true><<<g, 256, 0, h->stream>>>(rs, x, xstride, n, h->n_in, h->d_out, h->out_stride, h->scale);
+        else txfront_rot_kernel<false><<<g, 256, 0, h->stream>>>(rs, x, xstride, n, h->n_in, h->d_out, h->out_stride, h->scale);
+        h->launches++;
+    } else {
+        const int TM = h->G * TXF_R * h->P;
+        dim3 g(static_cast<unsigned>((n + TM - 1) / TM), h->C);
+        const unsigned nthr = static_cast<unsigned>(h->N * h->G);
+        if (sc16)
+            txfront_interp_kernel<TXF_R, true><<<g, nthr, h->smem, h->stream>>>(rs, x, xstride, n, h->n_in, h->d_hist[h->hist_cur], h->d_taps, h->N, h->NTP,
+                                                                              h->G, h->P, h->d_out, h->out_stride, h->scale);
+        else
+            txfront_interp_kernel<TXF_R, false><<<g, nthr, h->smem, h->stream>>>(rs, x, xstride, n, h->n_in, h->d_hist[h->hist_cur], h->d_taps, h->N, h->NTP,
+                                                                               h->G, h->P, h->d_out, h->out_stride, h->scale);
+        dim3 gh((h->H + 127) / 128, h->C);
+        frontend_hist_kernel<<<gh, 128, 0, h->stream>>>(rs, x, xstride, n, h->n_in, h->d_hist[h->hist_cur], h->d_hist[h->hist_cur ^ 1], h->H);
+        h->launches += 2;
+        h->hist_cur ^= 1;
+    }
+    h->n_in += n;
+    h->n_out_last = static_cast<long>(n * h->N);
+    if (n_out) *n_out = h->n_out_last;
+    CK(cudaGetLastError());
+    return QRL_OK;
+}
+int qrl_txfront_out_device(qrl_txfront* h, void** data, long* stride, long* n_out)
+{
+    if (!h) return QRL_EINVAL;
+    if (data) *data = h->d_out;
+    if (stride) *stride = static_cast<long>(h->out_stride);
+    if (n_out) *n_out = h->n_out_last;
+    return QRL_OK;
+}
+int qrl_txfront_read(qrl_txfront* h, void* dst, long cap)
+{
+    if (!h || !dst || cap < 0) return QRL_EINVAL;
+    const long w = std::min(cap, h->n_out_last);
+    const size_t isz = h->item_bytes();
+    if (w > 0) CK(cudaMemcpy2DAsync(dst, static_cast<size_t>(cap) * isz, h->d_out, static_cast<size_t>(h->out_stride) * isz, static_cast<size_t>(w) * isz, h->C, cudaMemcpyDeviceToHost, h->stream));
+    CK(cudaStreamSynchronize(h->stream));
+    return QRL_OK;
+}
+long qrl_txfront_launch_count(const qrl_txfront* h) { return h ? h->launches : 0; }
+
 // ---------------------------------------------------------------------------------------------- design helpers
 static int copy_out(const std::vector<float>& v, float* out, int cap, int per_item = 1)
 {

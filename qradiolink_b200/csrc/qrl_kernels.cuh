@@ -2835,6 +2835,117 @@ __global__ void frontend_hist_kernel(const RotState* __restrict__ rs, const floa
     new_hist[static_cast<long long>(c) * H + i] = v;
 }
 
+// ------------------------------------------------------------------------------------------------
+// TX front end (gr_mod_base.cpp:38,211-290): rotator_cc at 1 Msps, then rational_resampler_ccf(N, 1) up to the device rate
+//   y[N m + p] = sum_k arm[p][k] x[m - k],  arm[p][k] = h[p + k N],  one fmaf chain per output, oldest sample first.
+// grid = (tiles, channels); one CTA = P passes of G*R consecutive inputs of one channel, all N phases; thread (p = tid % N,
+// q = tid / N) owns phase p and R consecutive inputs per pass.  The taps sit in shared memory in chain order, row i = the taps of
+// step i ([NTP][N]: lanes on consecutive phases read consecutive words), the window holds the rotated samples (rotator fused into
+// the load, the previous calls' tail comes ALREADY ROTATED from `hist`, so a retune never reaches samples already in the filter).
+// Per step: one LDS (tap), one LDS.64 (the sample that slides into the R-slot register window), R FFMA2.  The arm is padded at
+// its oldest end to NTP = a multiple of R with zero taps: the chain starts at +0 and stays there through them, as the oracle's
+// own zero padding does, so the sums are the oracle's bit for bit.
+// Bound: 2 NTP lane-FMAs per output (NTP ~ 216 at every rate), FP32-pipe bound -- 148 SMs x 128 lanes / 432 per output; the
+// stores (8 B, or 4 B with SC16, per output) are an order of magnitude below the HBM write rate.
+// SC16: per component (short) clamp(rintf(v * scale), -32768, 32767), interleaved I/Q (a definition chosen here: the SIMD
+// fc32 -> sc16 converter's arithmetic, one multiply and round-half-even).
+__device__ __forceinline__ float2 txfront_rotate(const RotState& r, long long a, float2 v)
+{
+    const unsigned ph = r.base + r.inc * static_cast<unsigned>(a - r.n_base);
+    const float ang = static_cast<float>(static_cast<double>(static_cast<int>(ph)) * (3.14159265358979323846 / 2147483648.0));
+    float sn, cs;
+    qrl_sincosf(ang, sn, cs);
+    return make_float2(v.x * cs - v.y * sn, v.x * sn + v.y * cs);
+}
+__device__ __forceinline__ short txfront_sc16(float v, float scale)
+{
+    const float t = rintf(v * scale);
+    return static_cast<short>(t < -32768.0f ? -32768.0f : (t > 32767.0f ? 32767.0f : t));
+}
+template <bool SC16>
+__device__ __forceinline__ void txfront_store(void* out, long long i, float2 v, float scale)
+{
+    if (SC16) {
+        short2 s; s.x = txfront_sc16(v.x, scale); s.y = txfront_sc16(v.y, scale);
+        static_cast<short2*>(out)[i] = s;
+    } else static_cast<float2*>(out)[i] = v;
+}
+
+template <int R, bool SC16>
+__global__ void __launch_bounds__(256)
+txfront_interp_kernel(const RotState* __restrict__ rs /* nullptr: no rotation */, const float2* __restrict__ in, long long in_stride, long long T,
+                      long long n_abs0 /* absolute index of in[c][0] */, const float2* __restrict__ hist /* [C][H] rotated, H = NTP - 1 */,
+                      const float* __restrict__ taps /* [NTP][N] chain order */, int N, int NTP, int G, int P,
+                      void* __restrict__ out, long long out_stride /* items */, float scale)
+{
+    extern __shared__ __align__(16) float sm_txf[];
+    const int TM = G * R * P, H = NTP - 1;
+    float* hs = sm_txf;                                                 // NTP * N (rounded up to even)
+    float2* xs = reinterpret_cast<float2*>(sm_txf + ((NTP * N + 1) & ~1)); // TM + NTP - 1 rotated samples
+    const int c = blockIdx.y;
+    const long long t0 = static_cast<long long>(blockIdx.x) * TM;      // first input of the tile, relative to this call
+    const int nin = (T - t0) < TM ? static_cast<int>(T - t0) : TM;
+    const int nthr = N * G;
+    for (int i = threadIdx.x; i < NTP * N; i += nthr) hs[i] = taps[i];
+    const float2* x = in + static_cast<long long>(c) * in_stride;
+    const float2* hc = hist + static_cast<long long>(c) * H;
+    RotState r{ 0u, 0u, 0 };
+    if (rs) r = rs[c];
+    for (int i = threadIdx.x; i < TM + NTP - 1; i += nthr) {
+        const long long li = t0 - H + i;                               // index into this call's input
+        float2 v = make_float2(0.0f, 0.0f);
+        if (li >= 0) {
+            if (li < T) {
+                v = x[li];
+                if (rs) v = txfront_rotate(r, n_abs0 + li, v);
+            }
+        } else v = hc[H + li];
+        xs[i] = v;
+    }
+    __syncthreads();
+    const int p = threadIdx.x % N, q = threadIdx.x / N;
+    for (int ps = 0; ps < P; ps++) {
+        const int mi = (ps * G + q) * R;                                // tile-relative first input of this thread's R outputs
+        if (mi >= nin) break;
+        const float2* s = xs + mi;                                      // s[t] = x[t0 + mi - H + t]
+        float2 acc[R], w[R];
+#pragma unroll
+        for (int u = 0; u < R; u++) acc[u] = make_float2(0.0f, 0.0f);
+#pragma unroll
+        for (int u = 0; u < R - 1; u++) w[u] = s[u];
+        for (int i0 = 0; i0 < NTP; i0 += R) {
+#pragma unroll
+            for (int u = 0; u < R; u++) {
+                // step i = i0 + u: output j takes x[m_j - (NTP - 1 - i)] = s[i + j], which sits in slot (u + j) % R
+                w[(u + R - 1) % R] = s[i0 + u + R - 1];
+                const float h = hs[(i0 + u) * N + p];
+#pragma unroll
+                for (int j = 0; j < R; j++) ffma2(acc[j], h, w[(u + j) % R]);
+            }
+        }
+        const long long ob = static_cast<long long>(c) * out_stride + (t0 + mi) * N + p;
+#pragma unroll
+        for (int j = 0; j < R; j++)
+            if (mi + j < nin) txfront_store<SC16>(out, ob + static_cast<long long>(j) * N, acc[j], scale);
+    }
+}
+
+// N = 1 (device rate 1 Msps: the reference's rotator feeds the sink directly): rotation and the output format only
+template <bool SC16>
+__global__ void __launch_bounds__(256)
+txfront_rot_kernel(const RotState* __restrict__ rs, const float2* __restrict__ in, long long in_stride, long long T, long long n_abs0,
+                   void* __restrict__ out, long long out_stride, float scale)
+{
+    const int c = blockIdx.y;
+    RotState r{ 0u, 0u, 0 };
+    if (rs) r = rs[c];
+    for (long long i = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x; i < T; i += static_cast<long long>(gridDim.x) * blockDim.x) {
+        float2 v = in[static_cast<long long>(c) * in_stride + i];
+        if (rs) v = txfront_rotate(r, n_abs0 + i, v);
+        txfront_store<SC16>(out, static_cast<long long>(c) * out_stride + i, v, scale);
+    }
+}
+
 // roll the stage-1 history: new_hist = last H samples of (old_hist ++ iq[0..T))
 __global__ void hist_update_kernel(const float2* __restrict__ iq, long long iq_stride, long long T,
                                    const float2* __restrict__ old_hist, float2* __restrict__ new_hist, int H)

@@ -93,6 +93,14 @@ SYMBOLS = {
     "qrl_frontend_out_device": (_i, [_vp, C.POINTER(_vp), C.POINTER(_l), C.POINTER(_l)]),
     "qrl_frontend_read": (_i, [_vp, _vp, _l]),
     "qrl_frontend_launch_count": (_l, [_vp]),
+    "qrl_txfront_create": (_i, [_i, _i, _l, _i, C.c_float, _i, C.POINTER(_vp)]),
+    "qrl_txfront_destroy": (_i, [_vp]),
+    "qrl_txfront_set_stream": (_i, [_vp, _vp]),
+    "qrl_txfront_set_carrier_offset": (_i, [_vp, _i, _d]),
+    "qrl_txfront_work": (_i, [_vp, _vp, _l, _l, _i, C.POINTER(_l)]),
+    "qrl_txfront_out_device": (_i, [_vp, C.POINTER(_vp), C.POINTER(_l), C.POINTER(_l)]),
+    "qrl_txfront_read": (_i, [_vp, _vp, _l]),
+    "qrl_txfront_launch_count": (_l, [_vp]),
     "qrl_firdes_low_pass": (_i, [_d] * 4 + [_i, _vp, _i]),
     "qrl_firdes_low_pass_2": (_i, [_d] * 5 + [_i, _vp, _i]),
     "qrl_firdes_band_pass": (_i, [_d] * 5 + [_i, _vp, _i]),
